@@ -6,7 +6,7 @@ One STEP = the droid_backends work of one FactorGraph.update (SURVEY.md section 
 corr_index_forward over all edges + ba(iterations=2, lm=1e-4, ep=0.1) on a synthetic 512-edge / 72-keyframe graph at
 48x64 (fp16 correlation volumes as in the live system).
 
-    python bench.py [--gpus N --steps K --warmup W] [--impl reference]
+    python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--dump-outputs DIR]
 
 * our arm: `value` times the step with all inputs resident in HBM, launched through the C ABI (ctypes); `e2e` goes
   through the pybind `droid_backends` API from pinned HOST buffers (per-step inputs H2D, BA results D2H inside the timed
@@ -80,10 +80,17 @@ def parse():
     ap.add_argument("--no-graph", action="store_true", help="launch the step eagerly instead of replaying a captured CUDA graph (N=1)")
     ap.add_argument("--dropin-lookup", action="store_true", help="time the step with the four drop-in corr_index_forward launches on reference-layout volumes (round-1 definition) instead of the fused one-launch lookup on tiled volumes")
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary kernels (update operator, volume build, altcorr, geometry, solve) timed for `rooflines`")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32): poses, disps, dx, dz of ba and "
+                         "a fixed sample (seed 0) of the correlation lookup; rank 0, --impl ours")
     args = ap.parse_args()
     select_config(args)
     if args.steps is None:
         args.steps = 400 if (args.config == "metric" and args.impl == "ours") else 20
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs is supported for --impl ours only")
     return args
 
 
@@ -312,6 +319,7 @@ def run_ours(args, rank, world, dev):
     barrier()
     clocks = sampler.stop()
     ms_total = t_beg.elapsed_time(t_end)
+    outputs = snapshot_outputs(d, engine, corr196 if FUSED else corr_out) if args.dump_outputs and rank == 0 else None
     # the dominant kernel on its own stream position: the four corr_index launches of a step, CUDA events around them
     evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
     for k in range(args.steps):
@@ -488,7 +496,34 @@ def run_ours(args, rank, world, dev):
         line["rooflines"] = extras["rooflines"]
     if world == 1 and not args.no_cpu_baseline and CFG_NAME in ("metric", "c2", "c4"):
         line["cpu_baseline"] = cpu_baseline(pb)
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
     print(json.dumps(line))
+
+
+CORR_SAMPLE = 4 << 20     # lookup values kept by --dump-outputs (16 MB as float32)
+
+
+def snapshot_outputs(d, engine, corr):
+    """host copies of what the last timed step computed: ba's in-place poses / disps and its dx / dz, and a fixed seeded sample of the
+    4-level lookup in the [E, 196, ht, wd] layout of CorrBlock.__call__ (the fused launch writes that layout, the drop-in launches
+    are concatenated into it)"""
+    out = {k: d[k].float().cpu() for k in ("poses", "disps")}
+    out["dx"], out["dz"] = engine.dx.float().cpu(), engine.dz.float().cpu()
+    if isinstance(corr, list):
+        corr = torch.cat([c.view(c.shape[0], 49, HT, WD) for c in corr], 1) if corr else None
+    if corr is not None:
+        flat = corr.reshape(-1)
+        idx = torch.randint(0, flat.numel(), (min(CORR_SAMPLE, flat.numel()),), generator=torch.Generator().manual_seed(0))
+        out["corr_sample"] = flat[idx.to(flat.device)].float().cpu()
+    return out
+
+
+def write_outputs(dirname, outputs):
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(dirname, name + ".npy"), t.numpy().astype(np.float32))
 
 
 def _time_ms(fn, iters=5, warm=2):
