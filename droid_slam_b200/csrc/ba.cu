@@ -839,15 +839,6 @@ __device__ __forceinline__ float lds_f32(uint32_t addr) {
 }
 __device__ __forceinline__ void sts_f32(uint32_t addr, float v) { asm volatile("st.shared.f32 [%0], %1;" ::"r"(addr), "f"(v) : "memory"); }
 
-// debug timeline (DBA_TC_TIMING build only): globaltimer stamps of one CTA's warp 0 / MMA thread
-#ifdef DBA_TC_TIMING
-__device__ unsigned long long g_tc_timing[8192];
-__device__ __forceinline__ unsigned long long tc_gtimer() { unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); return t; }
-#define TC_STAMP(cond, idx) do { if (cond) g_tc_timing[(idx)] = tc_gtimer(); } while (0)
-#else
-#define TC_STAMP(cond, idx) do {} while (0)
-#endif
-
 // PAIR mode (frames with 22..100 rows: dense graphs, edge-sharded ranks): the rows are cut into tiles of 10; CTA (frame, pair z) stacks
 // tile a in operand rows 0..63 and tile b in rows 64..127 over the SAME 32 pixels (the packed layout with a zero pixel offset for the
 // second half), so the one M = N = 128 product holds S_ba in its lower-left block and S_aa / S_bb on the diagonal (emitted only by
@@ -904,7 +895,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) ba_schur_tc_kernel(
   const int R6a = PAIR ? 6 * min(kPairTileRows, nrows - kPairTileRows * ta) : 6 * nrows;
   const int R6b = PAIR ? 6 * min(kPairTileRows, nrows - kPairTileRows * tb) : 6 * nrows;
   const int R6 = R6a;                                    // operand rows 0..R6-1: E rows, row R6: w  (PAIR: of the half, see R6h)
-  TC_STAMP(blockIdx.x == 0 && blockIdx.y == 20 && threadIdx.x == 0, 7);
   const bool packed = !PAIR && (R6 + 2 <= 64);          // two PIXEL halves of a 64-pixel chunk in operand rows 0..63 / 64..127
   const bool two_halves = PAIR || packed;                // operand rows 64..127 carry a second set of lines
   const int nhalf = packed ? 2 : 1;
@@ -947,13 +937,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) ba_schur_tc_kernel(
   __syncthreads();
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem_base = *tmem_base_smem;
-  const bool dbg = (blockIdx.x == 0 && blockIdx.y == 20);
-  const bool dbg0 = dbg && tid == 0;
-  (void)dbg0;
-  TC_STAMP(dbg0, 0);
-#ifdef DBA_TC_TIMING
-  if (dbg0) { g_tc_timing[1] = (unsigned long long)nchunks; g_tc_timing[2] = (unsigned long long)R6; }
-#endif
 
   if (warp == 8) {
     // ================= MMA issuer =================
@@ -962,11 +945,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) ba_schur_tc_kernel(
       const uint32_t d_g = tmem_base + 3 * 128;
       for (int c = 0; c < nchunks; c++) {
         const int os = c % kTcOpStages, slot = c % kTcAccSlots;
-        TC_STAMP(dbg, 4096 + 4 * c + 0);
         mbar_wait(full + os, (c / kTcOpStages) & 1);
-        TC_STAMP(dbg, 4096 + 4 * c + 1);
         if (c >= kTcAccSlots) mbar_wait(acc_empty + slot, ((c / kTcAccSlots) - 1) & 1);
-        TC_STAMP(dbg, 4096 + 4 * c + 2);
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         const uint32_t hi0 = op_base + (uint32_t)os * 2 * kTcOpBytes, lo0 = hi0 + kTcOpBytes;
         const uint32_t d = tmem_base + (uint32_t)(slot * 128);
@@ -978,7 +958,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) ba_schur_tc_kernel(
         }
         umma_commit(empty + os);          // the operand stage may be overwritten once these MMAs have read it
         umma_commit(acc_full + slot);     // ... and the chunk's hi hi^T is ready to be drained
-        TC_STAMP(dbg, 4096 + 4 * c + 3);
       }
       umma_commit(done);
     }
@@ -1080,15 +1059,11 @@ __global__ void __launch_bounds__(kTcThreads, 1) ba_schur_tc_kernel(
       return make_float4(v.x > 0.f ? rsqrtf(v.x) : 0.f, v.y > 0.f ? rsqrtf(v.y) : 0.f, v.z > 0.f ? rsqrtf(v.z) : 0.f, v.w > 0.f ? rsqrtf(v.w) : 0.f);
     };
     float4 Cn0 = load_c4(0, 0), Cn1 = packed ? load_c4(0, 1) : make_float4(0.f, 0.f, 0.f, 0.f);
-    TC_STAMP(dbg0, 3);
     for (int c = 0; c < nchunks; c++) {
-      TC_STAMP(dbg0, 16 + 8 * c + 0);
       asm volatile("cp.async.wait_group %0;" ::"n"(kTcRawStages - 2) : "memory");
       __syncwarp();                                          // this warp's copies of chunk c have landed
-      TC_STAMP(dbg0, 16 + 8 * c + 1);
       const int os = c % kTcOpStages;
       if (c >= kTcOpStages) mbar_wait(empty + os, ((c / kTcOpStages) - 1) & 1);
-      TC_STAMP(dbg0, 16 + 8 * c + 2);
       const uint32_t raw = raw_base + (uint32_t)(c % kTcRawStages) * kTcRawBytes + (uint32_t)warp * 2048 + (uint32_t)(lane >> 3) * 128 +
                            (uint32_t)piece * 16;
       const uint32_t ophi = op_base + (uint32_t)os * 2 * kTcOpBytes;
@@ -1113,20 +1088,15 @@ __global__ void __launch_bounds__(kTcThreads, 1) ba_schur_tc_kernel(
           asm volatile("st.shared.v4.f32 [%0], {%1,%2,%3,%4};" ::"r"(ophi + kTcOpBytes + op_off[i]), "f"(lo[0]), "f"(lo[1]), "f"(lo[2]), "f"(lo[3]) : "memory");
         }
       }
-      TC_STAMP(dbg0, 16 + 8 * c + 3);
       asm volatile("fence.proxy.async.shared::cta;" ::: "memory");         // generic-proxy stores -> visible to the tensor core
       __syncwarp();
       if (lane == 0) mbar_arrive(full + os);
-      TC_STAMP(dbg0, 16 + 8 * c + 4);
       issue(c + kTcRawStages - 1);
-      TC_STAMP(dbg0, 16 + 8 * c + 5);
       if (c >= 2) drain(c - 2);
-      TC_STAMP(dbg0, 16 + 8 * c + 6);
     }
     asm volatile("cp.async.wait_group 0;" ::: "memory");
     if (nchunks >= 2) drain(nchunks - 2);
     drain(nchunks - 1);
-    TC_STAMP(dbg0, 4);
 
     // ================= G = hi lo^T: through shared memory (the operand ring is idle now) so that G + G^T can be formed
     mbar_wait(done, 0);
@@ -1175,10 +1145,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) ba_schur_tc_kernel(
       }
     }
   }
-  TC_STAMP(dbg0, 5);
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
-  TC_STAMP(dbg0, 6);
   if (warp == 8) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
 }
 
@@ -1371,18 +1339,12 @@ extern "C" int dba_ba_build(const dba_ba_args* a) {
     const int px_per_cta2 = ((HW + 2) / 3 + kSgK - 1) / kSgK * kSgK;
     const int gx2 = (HW + px_per_cta2 - 1) / px_per_cta2;
     const int zsplit2 = std::max(1, std::min(32, (6 * 148 + eff_frames * gx2 - 1) / (eff_frames * gx2)));
-    static bool attr_set = false;
-    if (!attr_set) {
-      DBA_CHECK_CUDA(cudaFuncSetAttribute(ba_schur_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2), "schur gemm smem attr");
-      DBA_CHECK_CUDA(cudaFuncSetAttribute(ba_schur_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2), "schur smem attr");
-      DBA_CHECK_CUDA(cudaFuncSetAttribute(ba_schur_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcSmem), "schur tc smem attr");
-      DBA_CHECK_CUDA(cudaFuncSetAttribute(ba_schur_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcSmem), "schur tc pair smem attr");
-      attr_set = true;
-    }
-    // frames with at most 21 rows go to the tensor cores (needs 16-byte aligned pixel rows); DBA_SCHUR_SIMT=1 keeps the CUDA-core path
-    static const bool force_simt = (getenv("DBA_SCHUR_SIMT") != nullptr && getenv("DBA_SCHUR_SIMT")[0] == '1');
-    const bool use_tc = (HW % 4 == 0) && !force_simt;
-    int pair_rows_max = kTcRowsMax;                  // frames with more rows than this go to the SIMT kernel
+    if ((rc = kernel_setup((const void*)ba_schur_gemm_kernel, (int)smem2))) return rc;
+    if ((rc = kernel_setup((const void*)ba_schur_small_kernel, (int)smem2))) return rc;
+    if ((rc = kernel_setup((const void*)ba_schur_tc_kernel<false>, (int)kTcSmem))) return rc;
+    if ((rc = kernel_setup((const void*)ba_schur_tc_kernel<true>, (int)kTcSmem))) return rc;
+    // frames with at most 21 rows go to the tensor cores (needs 16-byte aligned pixel rows)
+    const bool use_tc = HW % 4 == 0;
     if (use_tc) {
       const int tiles64 = (HW + 63) / 64;
       const int chunks_tc = std::max(1, std::min(tiles64, (148 + eff_frames / 2) / eff_frames));     // one CTA per SM
@@ -1392,14 +1354,12 @@ extern "C" int dba_ba_build(const dba_ba_args* a) {
                                                            WS(int, L.off_edgeidx), HW, a->t0, L.P, px_per_cta_tc, WS(float, L.off_Eij),
                                                            WS(float, L.off_C), WS(float, L.off_w), WS(float, L.off_Ei), Hsys, bsys, WS(int, L.off_big));
       // frames with 22..100 rows (dense graphs, edge-sharded ranks): tile pairs over gridDim.z, whole pixel range per CTA; CTAs of
-      // frames outside that range (and pair indices beyond a frame's count) exit after the row-list build.  DBA_SCHUR_PAIR=0: SIMT kernel.
-      static const bool no_pair = (getenv("DBA_SCHUR_PAIR") != nullptr && getenv("DBA_SCHUR_PAIR")[0] == '0');
+      // frames outside that range (and pair indices beyond a frame's count) exit after the row-list build
       const int max_big = std::min(a->n_frames, a->n_edges / kTcRowsMax);     // a frame with 22+ rows has 21+ out-edges
-      if (!no_pair && max_big > 0)
+      if (max_big > 0)
         ba_schur_tc_kernel<true><<<dim3(1, max_big, kPairGridZ), kTcThreads, kTcSmem, st>>>(a->jj, WS(int, L.off_hdr), WS(int, L.off_kx), WS(int, L.off_rowptr),
                                                            WS(int, L.off_edgeidx), HW, a->t0, L.P, ((HW + 31) / 32) * 32, WS(float, L.off_Eij),
                                                            WS(float, L.off_C), WS(float, L.off_w), WS(float, L.off_Ei), Hsys, bsys, WS(int, L.off_big));
-      pair_rows_max = no_pair ? kTcRowsMax : kPairRowsMax;
     } else {
       ba_schur_small_kernel<<<dim3(gx1, a->n_frames, 1), kSgThreads, smem2, st>>>(a->jj, WS(int, L.off_hdr), WS(int, L.off_kx), WS(int, L.off_rowptr),
                                                            WS(int, L.off_edgeidx), HW, a->t0, L.P, px_per_cta1, WS(float, L.off_Eij),
@@ -1407,7 +1367,7 @@ extern "C" int dba_ba_build(const dba_ba_args* a) {
     }
     DBA_CHECK_LAUNCH("ba_schur<single>");
     ba_schur_gemm_kernel<<<dim3(gx2, a->n_frames, zsplit2), kSgThreads, smem2, st>>>(a->jj, WS(int, L.off_hdr), WS(int, L.off_kx), WS(int, L.off_rowptr),
-                                                                         WS(int, L.off_edgeidx), HW, a->t0, L.P, px_per_cta2, use_tc ? pair_rows_max : kSgRows, WS(float, L.off_Eij),
+                                                                         WS(int, L.off_edgeidx), HW, a->t0, L.P, px_per_cta2, use_tc ? kPairRowsMax : kSgRows, WS(float, L.off_Eij),
                                                                          WS(float, L.off_C), WS(float, L.off_w), WS(float, L.off_Ei), Hsys, bsys);
     DBA_CHECK_LAUNCH("ba_schur<multi>");
   }
@@ -1473,13 +1433,6 @@ extern "C" int dba_ba_p2p_signal(const dba_ba_args* a) {
   DBA_CHECK_LAUNCH("ba_p2p_signal");
   return DBA_OK;
 }
-
-#ifdef DBA_TC_TIMING
-extern "C" int dba_debug_tc_timing(unsigned long long* out, int n) {
-  cudaDeviceSynchronize();
-  return (int)cudaMemcpyFromSymbol(out, dba::g_tc_timing, sizeof(unsigned long long) * (size_t)std::min(n, 8192));
-}
-#endif
 
 extern "C" int dba_ba(const dba_ba_args* a, int iterations) {
   int rc = dba_ba_prepare(a);

@@ -34,8 +34,6 @@
 #include <cooperative_groups.h>
 #include <math.h>
 #include <stdint.h>
-#include <stdlib.h>
-#include <string.h>
 
 namespace cg = cooperative_groups;
 
@@ -46,8 +44,6 @@ constexpr int kTP = kT + 1;            // padded row length in shared memory
 constexpr int kCholThreads = 256;      // 8 warps per CTA
 constexpr int kCholWarps = kCholThreads / 32;
 
-__device__ __forceinline__ unsigned long long gtimer() { unsigned long long t; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t)); return t; }
-#define CHOL_STAMP(slot) do { if (p.timing && cta == 0 && tid == 0) p.timing[(slot)] = gtimer(); } while (0)
 __device__ __forceinline__ double ldcg(const double* p) { return __ldcg(p); }
 __device__ __forceinline__ void stcg(double* p, double v) { __stcg(p, v); }
 
@@ -150,17 +146,13 @@ struct CholParams {
   double* L;         // [(nt+1)*32][nt*32] row-major working matrix (tile row nt carries b^T in its row 0)
   double* Linv;      // [nt][32][32] inverses of the diagonal tiles
   double* rdiag;     // [nt*32] reciprocals of diag(L)
-  int* first;        // [nt+1] envelope: first nonzero tile column of each tile row (rhs row nt: 0)
-  int* flags;        // (unused)
-  unsigned sleep_urgent, sleep_idle;   // resident-tile kernel: ns between polls of a warp on / off the critical path
-  int warm;                            // bit 1: the diagonal owner substitutes tile (j, j-1) itself (default; DBA_CHOL_FUSED_SUBST=0 turns it off)
-  double* Cs;                          // resident-tile kernel: [nt][32][32] tiles (j+1, j) BEFORE the substitution (for mode 2)
+  int* first;        // [nt+2] envelope: first nonzero tile column of each tile row (rhs row nt: 0); [nt+1]: spare word
+  double* Cs;                          // resident-tile kernel: [nt][32][32] tiles (j+1, j) BEFORE the substitution
   unsigned char map_i[128], map_j[128];   // resident-tile kernel: tile (i, j) of warp slot cta*8 + warp; 0xFF = none
   int* fail;         // sticky flag: non-positive pivot
   float* x;          // [n] result (fp32 like the reference's dx)
   int n, nt;
   double lm, ep;
-  unsigned long long* timing;   // debug (DBA_CHOL_TIMING=1): globaltimer stamps of CTA 0 / the potrf warp, else nullptr
   CholPeers peers;              // world <= 1: plain local system
 };
 
@@ -199,7 +191,7 @@ __device__ __forceinline__ void warp_tile_update(const double* At, const double*
   __syncwarp();
 }
 
-// Cluster-wide barrier WITHOUT the acquire side of barrier.cluster.wait.  Measured on B200 (this kernel, %globaltimer): every acquire --
+// Cluster-wide barrier WITHOUT the acquire side of barrier.cluster.wait.  Measured on B200 (this kernel, in-kernel timer stamps): every acquire --
 // barrier.cluster.wait, ld.acquire, fence -- ends in CCTL.IVALL, and the first global loads a warp issues after it take ~3 us instead of
 // ~0.3.  All data exchanged through this barrier is written with st.global.cg and read with ld.global.cg (L2 on both sides), so no L1
 // line ever has to be invalidated: every thread drains its own stores to L2 with a release store (MEMBAR.ALL.GPU, no CCTL), the CTA
@@ -333,9 +325,7 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_cluster_kernel(CholParam
       }
     }
   }
-  CHOL_STAMP(0);
   cluster.sync();
-  CHOL_STAMP(1);
 
   // ---- potrf of tile (0,0) --------------------------------------------------------------------------------------
   if (gw == 0) {
@@ -348,7 +338,6 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_cluster_kernel(CholParam
     stcg(p.rdiag + lane, rd);
   }
   cluster_sync_light(mbar, mphase, ncta, tid, drain);
-  CHOL_STAMP(2);
 
   for (int k = 0; k < nt; k++) {
     // ---- every CTA: L_kk and its reciprocal diagonal into shared memory
@@ -371,7 +360,6 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_cluster_kernel(CholParam
     }
     __syncthreads();
     const int nact = envelope ? s_nact : (nt - k);       // >= 1: the rhs row
-    CHOL_STAMP(8 + 8 * k + 0);
     // ---- TRSM: tiles (i,k) of the active rows (tile row nt is the right-hand side)
     for (int ta = gw; ta < nact; ta += nwarps) {
       const int i = envelope ? s_act[ta] : k + 1 + ta;
@@ -398,9 +386,7 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_cluster_kernel(CholParam
       for (int r = 0; r < kT; r++) stcg(tile + (size_t)r * ld + lane, s_A[warp][r][lane]);
       __syncwarp();
     }
-    CHOL_STAMP(8 + 8 * k + 1);
     cluster_sync_light(mbar, mphase, ncta, tid, drain);
-    CHOL_STAMP(8 + 8 * k + 2);
     // ---- trailing update with panel k
     const int rem = nt - k - 1;                       // remaining tile columns
     const int m1 = nact - 1;                          // active rows without the rhs row
@@ -434,13 +420,11 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_cluster_kernel(CholParam
       }
       __syncthreads();
       if (warp == 0) {
-        if (p.timing && lane == 0) p.timing[8 + 8 * k + 5] = gtimer();
         double a[kT], rd;
 #pragma unroll
         for (int c = 0; c < kT; c++) a[c] = s_T[lane][c];
         __syncwarp();
         if (!warp_potrf_compact(a, lane, s_col, s_T, rd) && lane == 0) *p.fail = 1;   // writes L into s_T
-        if (p.timing && lane == 0) p.timing[8 + 8 * k + 6] = gtimer();
         __syncwarp();
 #pragma unroll 8
         for (int r = 0; r < kT; r++) stcg(Ct + (size_t)r * ld + lane, s_T[r][lane]);
@@ -462,7 +446,6 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_cluster_kernel(CholParam
                          s_A[warp], s_B[warp]);
       }
     }
-    CHOL_STAMP(8 + 8 * k + 3);
     // inverse of L_kk (for the backward substitution) by the last warp of the cluster: lane j owns column j
     if (gw == nwarps - 1) {
       double xcol[kT];
@@ -477,7 +460,6 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_cluster_kernel(CholParam
       for (int i = 0; i < kT; i++) stcg(p.Linv + ((size_t)k * kT + i) * kT + lane, xcol[i]);
     }
     cluster_sync_light(mbar, mphase, ncta, tid, drain);
-    CHOL_STAMP(8 + 8 * k + 4);
   }
 
   if (cta != 0) return;
@@ -503,7 +485,6 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_cluster_kernel(CholParam
     }
     __syncthreads();
   }
-  CHOL_STAMP(3);
   const bool failed = (*reinterpret_cast<volatile int*>(p.fail)) != 0;
   for (int i = tid; i < n; i += kCholThreads) {
     const double v = ldcg(y + i);
@@ -516,7 +497,7 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_cluster_kernel(CholParam
 // Resident-tile dataflow variant for nt <= 14 (n <= 448: every frontend window, the 72-keyframe metric window).
 //
 // The barrier version above spends a panel on  L_kk reload -> TRSM -> cluster barrier -> trailing update -> cluster barrier.  Measured
-// (in-kernel %globaltimer): the arithmetic is ~3 us of that; the rest is synchronisation -- in particular every acquire (cluster barrier,
+// (in-kernel timer stamps): the arithmetic is ~3 us of that; the rest is synchronisation -- in particular every acquire (cluster barrier,
 // ld.acquire, fence) ends in CCTL.IVALL, after which the next global loads of the warp take ~3 us instead of ~0.3.
 // Here every lower tile (i,j) and every 32-entry piece of the right-hand side has ONE owner warp for the whole factorisation (105 + 14
 // tiles <= 128 warps of the 16-CTA cluster) and lives in that warp's registers.  An owner applies  C -= L_ik L_jk^T  for k = 0..j-1 as
@@ -529,6 +510,8 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_cluster_kernel(CholParam
 // Waits are bounded; a wait that expires marks the solve failed (dx = 0) instead of hanging.
 constexpr int kResMaxNt = 14;
 constexpr unsigned long long kSentinel = 0xFFF7DEADBEEF5A5Aull;
+constexpr unsigned kSleepUrgent = 300;    // ns between the polls of a warp on the critical path
+constexpr unsigned kSleepIdle = 4000;     // ... and of a warp off it
 
 
 __device__ __forceinline__ bool is_sentinel(double v) { return __double2hiint(v) == (int)(kSentinel >> 32); }   // arithmetic NaNs are canonical
@@ -598,8 +581,6 @@ __device__ __forceinline__ size_t sys_index(int r, int c, int n, bool diag_tile)
   }
   return (size_t)-1;
 }
-
-#define RES_STAMP(col, slot) do { if (p.timing && lane == 0) p.timing[8 + 16 * (col) + (slot)] = gtimer(); } while (0)
 
 template <bool PEERS>
 __global__ void __launch_bounds__(kCholThreads, 1) chol_resident_kernel(CholParams p) {
@@ -679,7 +660,7 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_resident_kernel(CholPara
     double* tile = L + (size_t)(i * kT) * ld + j * kT;
 #pragma unroll 8
     for (int r = 0; r < kT; r++) stcg(tile + (size_t)r * ld + lane, sentinel());
-    if (i == j + 1 && (p.warm & 2)) {
+    if (i == j + 1) {
 #pragma unroll 8
       for (int r = 0; r < kT; r++) stcg(p.Cs + ((size_t)j * kT + r) * kT + lane, sentinel());
     }
@@ -703,7 +684,6 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_resident_kernel(CholPara
   }
   __threadfence();
   cluster.sync();
-  if (p.timing && cta == 0 && tid == 0) p.timing[0] = p.timing[1] = p.timing[2] = gtimer();
 
   if (has_tile) {
     double (*sA)[kTP] = s_A[warp];
@@ -714,18 +694,16 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_resident_kernel(CholPara
       // ---------------- matrix tile (i, j): updates with the finished columns k < j
       for (int k = 0; k < j && alive; k++) {
         const bool last = (i == j && k == j - 1);
-        if (last) RES_STAMP(j, 8);
-        if (last && (p.warm & 2)) {
-          // mode 2: the diagonal owner does not wait for tile (j, j-1) to come back from its owner; it takes that tile as it was BEFORE
+        if (last) {
+          // the diagonal owner does not wait for tile (j, j-1) to come back from its owner; it takes that tile as it was BEFORE
           // the substitution (published early, off the critical path), substitutes against L_{j-1,j-1} itself and updates: one hand-over
           // per column instead of two.  The owner of (j, j-1) does the same substitution for everybody else.
-          alive = tile_fetch(p.Cs + (size_t)(j - 1) * kT * kT, kT, lane, sA, p.sleep_urgent, p.sleep_urgent);
-          alive = tile_fetch(L + (size_t)((j - 1) * kT) * ld + (j - 1) * kT, ld, lane, sB, p.sleep_urgent, p.sleep_urgent) && alive;
+          alive = tile_fetch(p.Cs + (size_t)(j - 1) * kT * kT, kT, lane, sA, kSleepUrgent, kSleepUrgent);
+          alive = tile_fetch(L + (size_t)((j - 1) * kT) * ld + (j - 1) * kT, ld, lane, sB, kSleepUrgent, kSleepUrgent) && alive;
           double rdl;
-          alive = vec_fetch(p.rdiag + (j - 1) * kT, lane, rdl, p.sleep_urgent) && alive;
+          alive = vec_fetch(p.rdiag + (j - 1) * kT, lane, rdl, kSleepUrgent) && alive;
           s_rd[warp][lane] = rdl;
           __syncwarp();
-          RES_STAMP(j, 9);
           double x[kT];
 #pragma unroll
           for (int c = 0; c < kT; c++) x[c] = sA[lane][c];
@@ -742,20 +720,17 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_resident_kernel(CholPara
           for (int c = 0; c < kT; c++) sA[lane][c] = x[c];
           __syncwarp();
           slab_mac(acc, sA, sA, lane);
-          RES_STAMP(j, 10);
           __syncwarp();
           continue;
         }
         const bool urgent = (i <= j + 1) && (k >= j - 2);     // the tile is (about to be) on the critical path
-        const unsigned slp = urgent ? p.sleep_urgent : p.sleep_idle;
-        alive = tile_fetch(L + (size_t)(i * kT) * ld + k * kT, ld, lane, sA, slp, p.sleep_urgent);
+        const unsigned slp = urgent ? kSleepUrgent : kSleepIdle;
+        alive = tile_fetch(L + (size_t)(i * kT) * ld + k * kT, ld, lane, sA, slp, kSleepUrgent);
         if (i != j) {
-          alive = tile_fetch(L + (size_t)(j * kT) * ld + k * kT, ld, lane, sB, slp, p.sleep_urgent) && alive;
+          alive = tile_fetch(L + (size_t)(j * kT) * ld + k * kT, ld, lane, sB, slp, kSleepUrgent) && alive;
           slab_mac(acc, sA, sB, lane);
         } else {
-          if (last) RES_STAMP(j, 9);
           slab_mac(acc, sA, sA, lane);
-          if (last) RES_STAMP(j, 10);
         }
         __syncwarp();
       }
@@ -771,18 +746,13 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_resident_kernel(CholPara
       for (int c = 0; c < kT; c++) a[c] = sA[lane][c];                 // lane = row
       __syncwarp();
       if (i == j) {
-        RES_STAMP(j, 0);
-        const long long ck0 = clock64();
         double rd;
         if (!warp_potrf_compact(a, lane, s_colb[warp], sA, rd) && lane == 0) *p.fail = 1;
         s_rd[warp][lane] = rd;
         __syncwarp();
-        RES_STAMP(j, 7);
-        if (p.timing && lane == 0) p.timing[8 + 16 * j + 13] = (unsigned long long)(clock64() - ck0);
         stcg(p.rdiag + j * kT + lane, rd);
 #pragma unroll 8
         for (int r = 0; r < kT; r++) stcg(tile + (size_t)r * ld + lane, sA[r][lane]);
-        RES_STAMP(j, 1);
         // inverse of L_jj for the backward pass (off the critical path), rolled: lane c owns column c of X = L^-1, kept in the warp's
         // second slab;  X[r][c] = (delta_rc - sum_{m<r} L[r][m] X[m][c]) / L[r][r]  (entries above the diagonal come out as zeros)
 #pragma unroll 1
@@ -798,18 +768,16 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_resident_kernel(CholPara
         for (int r = 0; r < kT; r++) stcg(p.Linv + ((size_t)j * kT + r) * kT + lane, sB[r][lane]);
       } else {
         const bool sub = (i == j + 1);
-        if (sub && (p.warm & 2)) {
+        if (sub) {
 #pragma unroll 8
           for (int r = 0; r < kT; r++) stcg(p.Cs + ((size_t)j * kT + r) * kT + lane, sA[r][lane]);
         }
-        if (sub) RES_STAMP(j, 2);
         double rdl;
-        const unsigned slp = sub ? p.sleep_urgent : p.sleep_idle;
-        alive = tile_fetch(L + (size_t)(j * kT) * ld + j * kT, ld, lane, sB, slp, p.sleep_urgent) && alive;
-        alive = vec_fetch(p.rdiag + j * kT, lane, rdl, p.sleep_urgent) && alive;
+        const unsigned slp = sub ? kSleepUrgent : kSleepIdle;
+        alive = tile_fetch(L + (size_t)(j * kT) * ld + j * kT, ld, lane, sB, slp, kSleepUrgent) && alive;
+        alive = vec_fetch(p.rdiag + j * kT, lane, rdl, kSleepUrgent) && alive;
         s_rd[warp][lane] = rdl;
         __syncwarp();
-        if (sub) RES_STAMP(j, 4);
 #pragma unroll
         for (int c = 0; c < kT; c++) {
           const double xv = a[c] * s_rd[warp][c];
@@ -818,20 +786,18 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_resident_kernel(CholPara
           for (int jj = c + 1; jj < kT; jj++) a[jj] -= xv * sB[jj][c];
           asm volatile("" ::: "memory");
         }
-        if (sub) RES_STAMP(j, 5);
 #pragma unroll
         for (int c = 0; c < kT; c++) sA[lane][c] = a[c];
         __syncwarp();
 #pragma unroll 8
         for (int r = 0; r < kT; r++) stcg(tile + (size_t)r * ld + lane, sA[r][lane]);
-        if (sub) RES_STAMP(j, 3);
       }
     } else {
       // ---------------- right-hand side piece j: lane c holds entry 32 j + c;  y_j = L_jj^-1 (b_j - sum_k L_jk y_k)
       for (int k = 0; k < j && alive; k++) {
         double yk;
-        alive = vec_fetch(yrow + k * kT, lane, yk, p.sleep_idle);
-        alive = tile_fetch(L + (size_t)(j * kT) * ld + k * kT, ld, lane, sA, p.sleep_idle, p.sleep_urgent) && alive;
+        alive = vec_fetch(yrow + k * kT, lane, yk, kSleepIdle);
+        alive = tile_fetch(L + (size_t)(j * kT) * ld + k * kT, ld, lane, sA, kSleepIdle, kSleepUrgent) && alive;
         double s0 = 0.0, s1 = 0.0;
 #pragma unroll
         for (int c = 0; c < kT; c += 2) {
@@ -842,8 +808,8 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_resident_kernel(CholPara
         __syncwarp();
       }
       double rdl;
-      alive = tile_fetch(L + (size_t)(j * kT) * ld + j * kT, ld, lane, sB, j == nt - 1 ? p.sleep_urgent : p.sleep_idle, p.sleep_urgent) && alive;
-      alive = vec_fetch(p.rdiag + j * kT, lane, rdl, p.sleep_urgent) && alive;
+      alive = tile_fetch(L + (size_t)(j * kT) * ld + j * kT, ld, lane, sB, j == nt - 1 ? kSleepUrgent : kSleepIdle, kSleepUrgent) && alive;
+      alive = vec_fetch(p.rdiag + j * kT, lane, rdl, kSleepUrgent) && alive;
 #pragma unroll
       for (int c = 0; c < kT; c++) {
         const double yc = __shfl_sync(0xffffffffu, y, c) * __shfl_sync(0xffffffffu, rdl, c);
@@ -851,7 +817,6 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_resident_kernel(CholPara
         else if (lane > c) y -= sB[lane][c] * yc;
       }
       stcg(yrow + j * kT + lane, y);
-      RES_STAMP(j, 11);
     }
     if (!alive && lane == 0) *p.fail = 4;                    // a producer never arrived: give up loudly, never hang
   }
@@ -882,7 +847,6 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_resident_kernel(CholPara
 #pragma unroll
     for (int r = 0; r < kT; r++) inv_c[r] = __ldcg(p.Linv + ((size_t)(nt - 1) * kT + r) * kT + lane);
     __syncthreads();
-    if (p.timing && tid == 0) p.timing[4] = gtimer();
     for (int k = nt - 1; k >= 0; k--) {
       const double* invp = p.Linv + (size_t)k * kT * kT + lane;
       if (k > 0) {
@@ -916,7 +880,6 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_resident_kernel(CholPara
       s_y[k * kT + lane] = xk;
       asm volatile("bar.sync 1, %0;" ::"n"(kCholThreads) : "memory");
       asm volatile("bar.sync 2, %0;" ::"n"(kCholThreads) : "memory");
-      RES_STAMP(k, 12);
 #pragma unroll
       for (int r = 0; r < kT; r++) inv_c[r] = inv_n[r];
     }
@@ -962,7 +925,6 @@ __global__ void __launch_bounds__(kCholThreads, 1) chol_resident_kernel(CholPara
     }
   }
   __syncthreads();
-  if (p.timing && tid == 0) p.timing[3] = gtimer();
   const bool failed = (*reinterpret_cast<volatile int*>(p.fail)) != 0;
   for (int q = tid; q < n; q += kCholThreads) {
     const double v = s_y[q];
@@ -1007,11 +969,40 @@ static bool resident_tile_map(int nt, int ncta, unsigned char* map_i, unsigned c
   return true;
 }
 
+// CTAs of the resident kernel's cluster for nt tile rows: every tile needs its own warp and every diagonal tile its own CTA.
+// 0: the system is too large for the resident kernel.
+static int resident_cluster_size(int nt) {
+  if (nt > kResMaxNt) return 0;
+  const int tiles = nt * (nt + 1) / 2 + nt;
+  int rcs = 1;
+  while (rcs * kCholWarps < tiles || rcs < nt) rcs *= 2;
+  return rcs;
+}
+
+constexpr int kCholDynSmem = (2 * kCholWarps + 2) * kT * kTP * sizeof(double);
+
+// the largest cluster (16 CTAs, else 8) the device can run chol_cluster_kernel with
+int chol_cluster_probe() {
+  kernel_setup((const void*)chol_cluster_kernel, kCholDynSmem, true);    // a failure here is reported by the launch
+  int best = 8;
+  for (int cs = 16; cs >= 8; cs -= 8) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(cs); cfg.blockDim = dim3(kCholThreads); cfg.dynamicSmemBytes = kCholDynSmem;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = cs; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+    cfg.attrs = at; cfg.numAttrs = 1;
+    int nclusters = 0;
+    if (cudaOccupancyMaxActiveClusters(&nclusters, chol_cluster_kernel, &cfg) == cudaSuccess && nclusters >= 1) { best = cs; break; }
+  }
+  cudaGetLastError();
+  return best;
+}
+
 size_t chol_workspace_bytes(int n) {
   const size_t nt = (size_t)(n + kT - 1) / kT;
   const size_t ld = nt * kT;
   return ((nt + 1) * kT * ld + nt * kT * kT + nt * kT) * sizeof(double) + (nt + 2) * sizeof(int) + 256 +
-         (size_t)(kResMaxNt + 1) * kResMaxNt * sizeof(int) + (size_t)kResMaxNt * kT * kT * sizeof(double) + 256;
+         (size_t)kResMaxNt * kT * kT * sizeof(double) + 256;
 }
 
 // H [n][n] fp64, b [n] fp64 -> x [n] fp32; fail flag is a device int
@@ -1026,92 +1017,34 @@ int chol_solve_launch(const double* H, const double* b, int n, double lm, double
   p.Linv = p.L + (size_t)(p.nt + 1) * kT * ld;
   p.rdiag = p.Linv + (size_t)p.nt * kT * kT;
   p.first = reinterpret_cast<int*>(p.rdiag + (size_t)p.nt * kT);
-  p.flags = p.first + (p.nt + 2);
-  p.Cs = reinterpret_cast<double*>((reinterpret_cast<uintptr_t>(p.flags + (kResMaxNt + 1) * kResMaxNt) + 255) & ~(uintptr_t)255);
+  p.Cs = reinterpret_cast<double*>((reinterpret_cast<uintptr_t>(p.first + (p.nt + 2)) + 255) & ~(uintptr_t)255);
 
-  const size_t dyn_smem = ((size_t)2 * kCholWarps + 2) * kT * kTP * sizeof(double);
-  static int cluster_size = 0;
-  if (cluster_size == 0) {
-    cudaFuncSetAttribute(chol_cluster_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-    cudaFuncSetAttribute(chol_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn_smem);
-    cudaFuncSetAttribute(chol_resident_kernel<false>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-    cudaFuncSetAttribute(chol_resident_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn_smem);
-    cudaFuncSetAttribute(chol_resident_kernel<true>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-    cudaFuncSetAttribute(chol_resident_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn_smem);
-    int best = 8;
-    for (int cs = 16; cs >= 8; cs -= 8) {
-      cudaLaunchConfig_t cfg = {};
-      cfg.gridDim = dim3(cs); cfg.blockDim = dim3(kCholThreads); cfg.dynamicSmemBytes = dyn_smem;
-      cudaLaunchAttribute at[1];
-      at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = cs; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-      cfg.attrs = at; cfg.numAttrs = 1;
-      int nclusters = 0;
-      if (cudaOccupancyMaxActiveClusters(&nclusters, chol_cluster_kernel, &cfg) == cudaSuccess && nclusters >= 1) { best = cs; break; }
-    }
-    cudaGetLastError();
-    cluster_size = best;
-  }
-  // small systems do not need the whole cluster
-  int cs = cluster_size;
-  const int tiles_first_panel = p.nt * (p.nt + 1) / 2 + 1;
-  while (cs > 1 && (cs / 2) * kCholWarps - 1 >= tiles_first_panel) cs /= 2;
+  int rc;
+  if ((rc = kernel_setup((const void*)chol_cluster_kernel, kCholDynSmem, true))) return rc;
+  if ((rc = kernel_setup((const void*)chol_resident_kernel<false>, kCholDynSmem, true))) return rc;
+  if ((rc = kernel_setup((const void*)chol_resident_kernel<true>, kCholDynSmem, true))) return rc;
+  DeviceInfo dev;
+  if ((rc = device_info(&dev))) return rc;
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(cs); cfg.blockDim = dim3(kCholThreads); cfg.dynamicSmemBytes = dyn_smem; cfg.stream = st;
+  cfg.blockDim = dim3(kCholThreads); cfg.dynamicSmemBytes = kCholDynSmem; cfg.stream = st;
   cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = cs; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+  at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
   cfg.attrs = at; cfg.numAttrs = 1;
-  static unsigned long long* tbuf = nullptr;
-  static const bool want_timing = getenv("DBA_CHOL_TIMING") != nullptr;
-  p.timing = nullptr;
-  if (want_timing) {
-    if (!tbuf) cudaMallocHost(&tbuf, 4096 * sizeof(unsigned long long));
-    memset(tbuf, 0, 4096 * sizeof(unsigned long long));
-    if (8 + 16 * p.nt < 4096) p.timing = tbuf;
-  }
-  // resident-tile dataflow kernel: every tile needs its own warp
-  static const bool allow_resident = !(getenv("DBA_CHOL_RESIDENT") && atoi(getenv("DBA_CHOL_RESIDENT")) == 0);
-  const int res_tiles = p.nt * (p.nt + 1) / 2 + p.nt;
-  int rcs = 1;
-  while (rcs * kCholWarps < res_tiles || rcs < p.nt) rcs *= 2;
-  if (allow_resident && p.nt <= kResMaxNt && rcs <= cluster_size && resident_tile_map(p.nt, rcs, p.map_i, p.map_j)) {
+  const int rcs = resident_cluster_size(p.nt);
+  if (rcs > 0 && rcs <= dev.chol_cluster && resident_tile_map(p.nt, rcs, p.map_i, p.map_j)) {
     cfg.gridDim = dim3(rcs);
     at[0].val.clusterDim.x = rcs;
-    static const unsigned sl_u = getenv("DBA_CHOL_SLEEP_URGENT") ? (unsigned)atoi(getenv("DBA_CHOL_SLEEP_URGENT")) : 300u;
-    static const unsigned sl_i = getenv("DBA_CHOL_SLEEP_IDLE") ? (unsigned)atoi(getenv("DBA_CHOL_SLEEP_IDLE")) : 4000u;
-    p.sleep_urgent = sl_u; p.sleep_idle = sl_i;
-    static const int warm = getenv("DBA_CHOL_FUSED_SUBST") ? (atoi(getenv("DBA_CHOL_FUSED_SUBST")) ? 2 : 0) : 2;
-    p.warm = warm;
     if (p.peers.world > 1) DBA_CHECK_CUDA(cudaLaunchKernelEx(&cfg, chol_resident_kernel<true>, p), "chol_resident_kernel launch");
     else DBA_CHECK_CUDA(cudaLaunchKernelEx(&cfg, chol_resident_kernel<false>, p), "chol_resident_kernel launch");
-    if (p.timing) {
-      cudaStreamSynchronize(st);
-      const unsigned long long t0 = tbuf[0];
-      fprintf(stderr, "[chol resident timing] n=%d nt=%d cluster=%d  factor+forward %.1f us, backsub %.1f us\n", n, p.nt, rcs, (tbuf[4] - t0) / 1e3,
-              (tbuf[3] - tbuf[4]) / 1e3);
-      for (int k = 0; k < p.nt; k++) {
-        const unsigned long long* q = tbuf + 8 + 16 * k;
-        auto d = [&](int a, int b) { return (q[a] && q[b]) ? (double)((long long)q[a] - (long long)q[b]) / 1e3 : 0.0; };
-        fprintf(stderr, "  column %2d: diag: last update starts@%.1f wait+load %.1f mac %.1f transpose %.1f potrf %.1f store %.1f | (k+1,k): ready %+.1f after that, wait+load L_kk %.1f subst %.1f store %.1f\n",
-                k, q[8] ? (q[8] - t0) / 1e3 : 0.0, d(9, 8), d(10, 9), d(0, 10), d(7, 0), d(1, 7), d(2, 1), d(4, 2), d(5, 4), d(3, 5));
-        fprintf(stderr, "             y piece stored@%.1f   backward step done@%.1f   potrf: %llu SM cycles in %.2f us = %.0f MHz\n", q[11] ? (q[11] - t0) / 1e3 : 0.0,
-                q[12] ? (q[12] - t0) / 1e3 : 0.0, q[13], d(7, 0), d(7, 0) > 0 ? (double)q[13] / d(7, 0) : 0.0);
-      }
-    }
     return DBA_OK;
   }
+  // small systems do not need the whole cluster
+  int cs = dev.chol_cluster;
+  const int tiles_first_panel = p.nt * (p.nt + 1) / 2 + 1;
+  while (cs > 1 && (cs / 2) * kCholWarps - 1 >= tiles_first_panel) cs /= 2;
+  cfg.gridDim = dim3(cs);
+  at[0].val.clusterDim.x = cs;
   DBA_CHECK_CUDA(cudaLaunchKernelEx(&cfg, chol_cluster_kernel, p), "chol_cluster_kernel launch");
-  if (p.timing) {
-    cudaStreamSynchronize(st);
-    const unsigned long long t0 = tbuf[0];
-    fprintf(stderr, "[chol timing] n=%d nt=%d cluster=%d  load %.1f us, potrf0 %.1f us, total-to-backsub-end %.1f us\n", n, p.nt, cs, (tbuf[1] - t0) / 1e3,
-            (tbuf[2] - tbuf[1]) / 1e3, (tbuf[3] - t0) / 1e3);
-    for (int k = 0; k < p.nt; k++) {
-      const unsigned long long* q = tbuf + 8 + 8 * k;
-      fprintf(stderr, "  panel %2d: Lkk-load@%.1f trsm(cta0) %.1f  barrier %.1f  update(cta0 thread0) %.1f  inv+barrier %.1f | diag tile: coop-update %.1f potrf %.1f\n", k,
-              (q[0] - t0) / 1e3, (q[1] - q[0]) / 1e3, (q[2] - q[1]) / 1e3, (q[3] - q[2]) / 1e3, (q[4] - q[3]) / 1e3,
-              q[5] ? (q[5] - q[2]) / 1e3 : 0.0, q[6] ? (q[6] - q[5]) / 1e3 : 0.0);
-    }
-  }
   return DBA_OK;
 }
 
@@ -1122,11 +1055,8 @@ int chol_solve_launch(const double* H, const double* b, int n, double lm, double
 extern "C" int dba_solve_tile_placement(int n, unsigned char* map_i, unsigned char* map_j) {
   if (n <= 0 || !map_i || !map_j) return 0;
   const int nt = (n + dba::kT - 1) / dba::kT;
-  if (nt > dba::kResMaxNt) return 0;
-  const int tiles = nt * (nt + 1) / 2 + nt;
-  int rcs = 1;
-  while (rcs * dba::kCholWarps < tiles || rcs < nt) rcs *= 2;
-  if (rcs > 16 || !dba::resident_tile_map(nt, rcs, map_i, map_j)) return 0;
+  const int rcs = dba::resident_cluster_size(nt);
+  if (rcs == 0 || !dba::resident_tile_map(nt, rcs, map_i, map_j)) return 0;
   return rcs;
 }
 

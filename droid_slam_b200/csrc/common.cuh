@@ -1,5 +1,6 @@
 // Shared device helpers for the sm_100a kernels of the dense-BA update path.
 #pragma once
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <cuda_fp16.h>
 #include <cuda_bf16.h>
@@ -10,8 +11,26 @@
 namespace dba {
 
 void set_error(const char* fmt, ...);
+
+// ---- per-device host setup (common.cu), keyed by the current device and safe to call from several threads --------------
+struct DeviceInfo {
+  int num_sms;
+  int smem_optin;       // cudaDevAttrMaxSharedMemoryPerBlockOptin
+  int chol_cluster;     // largest cluster (16 or 8 CTAs) chol_cluster_kernel can be launched with
+};
+// facts of the current device, gathered on its first use
+int device_info(DeviceInfo* out);
+// opts `kernel` into `smem_bytes` of dynamic shared memory (and into non-portable cluster sizes) on the current device; the
+// attribute is applied on the first call per device, so a kernel must always be passed the same values
+int kernel_setup(const void* kernel, int smem_bytes, bool nonportable_cluster = false);
+// cuTensorMapEncodeTiled through the runtime's driver entry point (no link-time dependency on libcuda); nullptr if unavailable
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
+                                  const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+EncodeTiledFn tensor_map_encoder();
+
 // chol.cu: damped SPD solve (fp64, one thread-block cluster)
 size_t chol_workspace_bytes(int n);
+int chol_cluster_probe();     // for device_info(): the cluster-size probe of chol_cluster_kernel on the current device
 struct CholPeers {            // fused peer-to-peer reduction (world > 1): H/b are summed over peer copies in rank order
   int world;
   const double* sys[8];       // peer-mapped pointers to each rank's [n*n + n] system for this epoch

@@ -235,23 +235,9 @@ __global__ void __launch_bounds__(kCvThreads, 1) corr_volume_pyramid_kernel(cons
   if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
 }
 
-// ---- host: tensor maps through the driver entry point (no link-time dependency on libcuda) ------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                                  const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeTiledFn get_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* ptr = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres) != cudaSuccess || qres != cudaDriverEntryPointSuccess) return nullptr;
-    fn = reinterpret_cast<EncodeTiledFn>(ptr);
-  }
-  return fn;
-}
-
+// ---- host -------------------------------------------------------------------------------------------------------------
 static int make_fmap_tensor_map(CUtensorMap* map, const void* base, int n_frames, int C, int HW) {
-  EncodeTiledFn enc = get_encode_fn();
+  EncodeTiledFn enc = tensor_map_encoder();
   if (!enc) { set_error("cuTensorMapEncodeTiled entry point not available"); return DBA_ERR_CUDA; }
   cuuint64_t dims[3] = {(cuuint64_t)HW, (cuuint64_t)C, (cuuint64_t)n_frames};
   cuuint64_t strides[2] = {(cuuint64_t)HW * 2, (cuuint64_t)HW * C * 2};       // bytes, dims 1..2
@@ -285,8 +271,7 @@ static int corr_volume_launch(const void* fmap1, const void* fmap2, const int64_
   CUtensorMap tmA, tmB;
   int rc = make_fmap_tensor_map(&tmA, fmap1, n_frames1, channels, HW); if (rc) return rc;
   rc = make_fmap_tensor_map(&tmB, fmap2, n_frames2, channels, HW); if (rc) return rc;
-  static bool attr = false;
-  if (!attr) { DBA_CHECK_CUDA(cudaFuncSetAttribute(corr_volume_pyramid_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kCvSmem), "corr_volume smem attr"); attr = true; }
+  rc = kernel_setup((const void*)corr_volume_pyramid_kernel, kCvSmem); if (rc) return rc;
   CvParams p;
   p.ii = ii; p.jj = jj; p.out0 = (__half*)out0; p.out1 = (__half*)out1; p.out2 = (__half*)out2; p.out3 = (__half*)out3;
   p.HW = HW; p.wd = wd; p.n_chunks = HW / kCvN; p.tiled = tiled;

@@ -196,13 +196,10 @@ extern "C" int dba_proximity_edges(const float* d, int t0, int t1, int t, const 
   p.t0 = t0; p.t1 = t1; p.t = t; p.rad = rad; p.nms = nms; p.max_factors = max_factors; p.stereo = stereo; p.thresh = thresh;
   p.es = reinterpret_cast<long long*>(es); p.cap = cap; p.hdr = hdr; p.bitmap_global = bitmap;
   const size_t bm_bytes = ((size_t)(n + 31) / 32) * 4;
-  static int max_smem = -1;
-  if (max_smem < 0) {
-    int dev = 0; cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-    max_smem -= 1024;
-    cudaFuncSetAttribute(prox_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
-  }
+  DeviceInfo dev;
+  int rc = device_info(&dev); if (rc) return rc;
+  const int max_smem = dev.smem_optin - 1024;
+  rc = kernel_setup((const void*)prox_select_kernel, max_smem); if (rc) return rc;
   p.bitmap_in_smem = bm_bytes <= (size_t)max_smem ? 1 : 0;
   prox_select_kernel<<<1, kProxThreads, p.bitmap_in_smem ? bm_bytes : 0, st>>>(p);
   DBA_CHECK_LAUNCH("prox_select");

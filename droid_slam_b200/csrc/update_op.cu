@@ -23,14 +23,12 @@
 #include "tcgen05.cuh"
 #include <cuda.h>
 #include <string.h>
-#include <stdlib.h>
 
 namespace dba {
 
 enum { EPI_STORE = 0, EPI_GATE = 1, EPI_ZR = 2, EPI_Q = 3, EPI_F32 = 4, EPI_NCHW = 5 };
 
 constexpr int kUpThreads = 320;   // warp 0 TMA, warp 1 MMA, warps 2..9 epilogue
-constexpr bool kPairDefault = false;   // cta_group::2 kernel by default
 
 struct ConvParams {
   int E, HT, WD;                    // images (edges or frames), image height / width
@@ -138,14 +136,13 @@ __device__ __forceinline__ float warp_column_sums(float (&v)[32], int lane) {
   return v[0];
 }
 
-// epilogue of one CTA tile (MT x 128 pixels x this warp's column range) out of the TMEM accumulator buffer `buf`; `store` = false
-// for the duplicated tile a CTA pair computes when the tile count is odd (everything is computed, nothing is written)
+// epilogue of one CTA tile (MT x 128 pixels x this warp's column range) out of the TMEM accumulator buffer `buf`
 template <int EPI>
 __device__ __forceinline__ void conv_epilogue_tile(const ConvParams& p, uint32_t tmem_base, uint32_t buf, int q, int lane, int c_begin, int c_end, int my, int mx,
-                                                   int nt, int e, int ty, int tx, bool store) {
+                                                   int nt, int e, int ty, int tx) {
   for (int t = 0; t < p.MT; t++) {
     const int y = ty * (p.MT * p.RM) + t * p.RM + my, x = tx * p.TW + mx;
-    const bool valid = store && y < p.HT && x < p.WD;
+    const bool valid = y < p.HT && x < p.WD;
     const size_t pix = ((size_t)e * p.HT + (valid ? y : 0)) * p.WD + (valid ? x : 0);
     for (int c0 = c_begin; c0 < c_end; c0 += 32) {
       uint32_t raw[32];
@@ -169,7 +166,7 @@ __device__ __forceinline__ void conv_epilogue_tile(const ConvParams& p, uint32_t
         for (int j = 0; j < 32; j++) v[j] = valid ? sigmoid_fast(v[j]) * hh[j] : 0.f;
         const float s = warp_column_sums(v, lane);
         const int slot = ((ty * p.tiles_x + tx) * p.MT + t) * 4 + q;
-        if (store) p.partial[((size_t)e * p.slots + slot) * 128 + c0 + lane] = s;
+        p.partial[((size_t)e * p.slots + slot) * 128 + c0 + lane] = s;
       } else if (EPI == EPI_ZR) {
         const float* g = p.glo + (size_t)e * 384 + c0;
 #pragma unroll
@@ -352,7 +349,7 @@ __global__ void __launch_bounds__(kUpThreads, 1) conv_tc_kernel(const __grid_con
       const uint32_t buf = it % p.nbuf;
       mbar_wait(tmem_full + buf, (it / p.nbuf) & 1);
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      conv_epilogue_tile<EPI>(p, tmem_base, buf, q, lane, c_begin, c_end, my, mx, nt, e, ty, tx, true);
+      conv_epilogue_tile<EPI>(p, tmem_base, buf, q, lane, c_begin, c_end, my, mx, nt, e, ty, tx);
       asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
       __syncwarp();
       if (lane == 0) mbar_arrive(tmem_empty + buf);
@@ -361,208 +358,6 @@ __global__ void __launch_bounds__(kUpThreads, 1) conv_tc_kernel(const __grid_con
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
   if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
-}
-
-// ---------------------------------------------------------------------------------------------------------------------------
-// CTA-pair variant (tcgen05 cta_group::2): two CTAs of a cluster (one SM pair) work on two CTA tiles at once and SHARE every weight
-// stage -- each CTA loads only half of the N weight rows, the pair-wide MMA (M = 256: CTA 0's 128 pixels + CTA 1's 128 pixels,
-// N = all output channels) reads both halves.  Per MMA a CTA's tensor core now fetches 4 KB of A + half of B from shared memory
-// instead of all of B (the single-CTA form is shared-memory-operand bound: 128 B/clk at N = 128), and the L2 -> SM weight traffic
-// per MAC halves.  The leader CTA (rank 0) issues all MMAs; both CTAs run their own TMA producer and their own epilogue on their
-// own TMEM lanes.  Barrier protocol (the usual 2-SM pipeline): "full" barriers live in the leader and collect both CTAs' loads
-// (the peer's TMA signals the leader's barrier; count 2 = leader arrive.expect_tx + peer arrive), "empty" / "tmem_full" barriers
-// live in each CTA and are released by one multicast tcgen05.commit, "tmem_empty" lives in the leader and collects all 16
-// epilogue warps.
-// ---------------------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ uint32_t mapa_rank(uint32_t smem_addr, uint32_t rank) {
-  uint32_t r; asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_addr), "r"(rank)); return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-__device__ __forceinline__ void tma2_load_4d(void* smem_dst, const CUtensorMap* map, uint32_t bar_cluster_addr, int c0, int c1, int c2, int c3) {
-  asm volatile("cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-               ::"r"(smem_u32(smem_dst)), "l"(map), "r"(bar_cluster_addr), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
-}
-__device__ __forceinline__ void tma2_load_3d(void* smem_dst, const CUtensorMap* map, uint32_t bar_cluster_addr, int c0, int c1, int c2) {
-  asm volatile("cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-               ::"r"(smem_u32(smem_dst)), "l"(map), "r"(bar_cluster_addr), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-__device__ __forceinline__ void umma2_commit_mc(uint64_t* bar) {      // arrive on this barrier in BOTH CTAs of the pair when the MMAs issued so far are done
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)), "h"((uint16_t)3) : "memory");
-}
-__device__ __forceinline__ void umma2_f16_ss(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-
-template <int EPI>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kUpThreads, 1) conv_tc2_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUtensorMap tmA1,
-                                                                                         const __grid_constant__ CUtensorMap tmW, const ConvParams p) {
-  extern __shared__ uint8_t up_smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(up_smem_raw) + 1023) & ~(uintptr_t)1023);
-  uint8_t* sA = smem;
-  uint8_t* sB = smem + p.a_stages * p.a_bytes;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sB + p.b_stages * p.b_bytes);       // b_bytes = this CTA's half of a weight stage
-  uint64_t* a_full = bars;              // [4]  used in the leader
-  uint64_t* a_empty = bars + 4;         // [4]
-  uint64_t* b_full = bars + 8;          // [8]  used in the leader
-  uint64_t* b_empty = bars + 16;        // [8]
-  uint64_t* tmem_full = bars + 24;      // [2]
-  uint64_t* tmem_empty = bars + 26;     // [2]  used in the leader
-  uint32_t* tmem_base_smem = reinterpret_cast<uint32_t*>(bars + 28);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const bool leader = rank == 0;
-  const int tiles_per_img = p.tiles_x * p.tiles_y;
-  const int tpn = p.E * tiles_per_img;                 // CTA tiles per N tile
-  const int ppn = (tpn + 1) >> 1;                      // pair tiles per N tile
-  const int total_pairs = p.n_ntiles * ppn;
-  const int npairs = gridDim.x >> 1, pair = blockIdx.x >> 1;
-  const int nk = p.nk0 + p.nk1;
-  const int pad = p.KS >> 1;
-  const int n_c0 = p.N > 256 ? 256 : p.N, n_c1 = p.N - n_c0;
-
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < p.a_stages; s++) { mbar_init(a_full + s, 2); mbar_init(a_empty + s, 1); }
-    for (int s = 0; s < p.b_stages; s++) { mbar_init(b_full + s, 2); mbar_init(b_empty + s, 1); }
-    for (int s = 0; s < 2; s++) { mbar_init(tmem_full + s, 1); mbar_init(tmem_empty + s, 16); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(smem_u32(tmem_base_smem)) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  cluster_sync_all();                                   // barriers of both CTAs initialised, TMEM of both allocated
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  const uint32_t tmem_base = *tmem_base_smem;
-
-  if (warp == 0) {
-    // ================= TMA producer (one thread per CTA): own halo tiles, own half of the weight rows =================
-    if (lane == 0) {
-      uint32_t ac = 0, bc = 0;
-      const int h0 = n_c0 >> 1, h1 = n_c1 >> 1;          // this CTA's rows of the two N chunks
-      for (int T = pair; T < total_pairs; T += npairs) {
-        const int nt = T / ppn;
-        int r0 = 2 * (T - nt * ppn) + (int)rank;
-        if (r0 >= tpn) r0 = tpn - 1;                     // odd tile count: the pair's second CTA recomputes the last tile (not stored)
-        const int e = r0 / tiles_per_img;
-        const int r1 = r0 - e * tiles_per_img;
-        const int ty = r1 / p.tiles_x, tx = r1 - ty * p.tiles_x;
-        const int y0 = ty * (p.MT * p.RM), x0 = tx * p.TW;
-        for (int kb = 0; kb < nk; kb++) {
-          const CUtensorMap* am = kb < p.nk0 ? &tmA0 : &tmA1;
-          const int ch = (kb < p.nk0 ? kb : kb - p.nk0) * 64;
-          for (int dx = 0; dx < p.KS; dx++) {
-            const int as = ac % p.a_stages;
-            mbar_wait(a_empty + as, ((ac / p.a_stages) & 1) ^ 1);
-            const uint32_t fa = mapa_rank(smem_u32(a_full + as), 0);
-            tma2_load_4d(sA + as * p.a_bytes, am, fa, ch, x0 + dx - pad, y0 - pad, e);
-            if (leader) mbar_expect_tx(a_full + as, 2 * p.a_bytes); else mbar_arrive_cluster(fa);
-            ac++;
-            for (int dy = 0; dy < p.KS; dy++) {
-              const int bs = bc % p.b_stages;
-              mbar_wait(b_empty + bs, ((bc / p.b_stages) & 1) ^ 1);
-              const uint32_t fb = mapa_rank(smem_u32(b_full + bs), 0);
-              uint8_t* dstb = sB + bs * p.b_bytes;
-              const int tap = dy * p.KS + dx;
-              for (int n = 0; n < h0; n += p.boxn) tma2_load_3d(dstb + n * 128, &tmW, fb, kb * 64, nt * p.N + (int)rank * h0 + n, tap);
-              for (int n = 0; n < h1; n += p.boxn) tma2_load_3d(dstb + (h0 + n) * 128, &tmW, fb, kb * 64, nt * p.N + n_c0 + (int)rank * h1 + n, tap);
-              if (leader) mbar_expect_tx(b_full + bs, 2 * p.b_bytes); else mbar_arrive_cluster(fb);
-              bc++;
-            }
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ================= MMA issuer: leader CTA only, M = 256 across the pair =================
-    if (leader) {
-      const uint32_t idesc0 = umma_idesc_f16_kk(256, n_c0);
-      const uint32_t idesc1 = n_c1 ? umma_idesc_f16_kk(256, n_c1) : 0u;
-      const uint32_t sA_u = smem_u32(sA), sB_u = smem_u32(sB);
-      uint32_t ac = 0, bc = 0, it = 0;
-      for (int T = pair; T < total_pairs; T += npairs, it++) {
-        const uint32_t buf = it % p.nbuf;
-        mbar_wait(tmem_empty + buf, ((it / p.nbuf) & 1) ^ 1);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        const uint32_t tcol = tmem_base + buf * 256;
-        bool first = true;
-        for (int kb = 0; kb < nk; kb++) {
-          for (int dx = 0; dx < p.KS; dx++) {
-            const int as = ac % p.a_stages;
-            mbar_wait(a_full + as, (ac / p.a_stages) & 1);
-            for (int dy = 0; dy < p.KS; dy++) {
-              const int bs = bc % p.b_stages;
-              mbar_wait(b_full + bs, (bc / p.b_stages) & 1);
-              asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-              if (lane == 0) {
-                const uint32_t b_base = sB_u + bs * p.b_bytes;
-                for (int t = 0; t < p.MT; t++) {
-                  const uint32_t a_base = sA_u + as * p.a_bytes + (uint32_t)((t * p.RM + dy) * p.TW) * 128u;
-#pragma unroll
-                  for (int k = 0; k < 4; k++) {
-                    const uint32_t acc = (first && k == 0) ? 0u : 1u;
-                    const uint64_t ad = umma_desc_k_sw128(a_base + k * 32, 1024);
-                    umma2_f16_ss(tcol + t * p.N, ad, umma_desc_k_sw128(b_base + k * 32, 1024), idesc0, acc);
-                    if (n_c1) umma2_f16_ss(tcol + t * p.N + 256, ad, umma_desc_k_sw128(b_base + (n_c0 >> 1) * 128 + k * 32, 1024), idesc1, acc);
-                  }
-                }
-                umma2_commit_mc(b_empty + bs);
-              }
-              __syncwarp();
-              first = false;
-              bc++;
-            }
-            if (lane == 0) umma2_commit_mc(a_empty + as);
-            __syncwarp();
-            ac++;
-          }
-        }
-        if (lane == 0) umma2_commit_mc(tmem_full + buf);
-        __syncwarp();
-      }
-    }
-  } else {
-    // ================= epilogue: every CTA drains its own 128 TMEM lanes =================
-    const int q = warp & 3;
-    const int half = (warp - 2) >> 2;
-    const int cols_per_half = p.N >= 64 ? p.N / 2 : p.N;
-    const int c_begin = half * cols_per_half;
-    const int c_end = (p.N >= 64 || half == 0) ? c_begin + cols_per_half : c_begin;
-    const int m = q * 32 + lane;
-    const int my = m / p.TW, mx = m - my * p.TW;
-    uint32_t it = 0;
-    for (int T = pair; T < total_pairs; T += npairs, it++) {
-      const int nt = T / ppn;
-      int r0 = 2 * (T - nt * ppn) + (int)rank;
-      const bool store = r0 < tpn;
-      if (!store) r0 = tpn - 1;
-      const int e = r0 / tiles_per_img;
-      const int r1 = r0 - e * tiles_per_img;
-      const int ty = r1 / p.tiles_x, tx = r1 - ty * p.tiles_x;
-      const uint32_t buf = it % p.nbuf;
-      mbar_wait(tmem_full + buf, (it / p.nbuf) & 1);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      conv_epilogue_tile<EPI>(p, tmem_base, buf, q, lane, c_begin, c_end, my, mx, nt, e, ty, tx, store);
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-      __syncwarp();
-      if (lane == 0) mbar_arrive_cluster(mapa_rank(smem_u32(tmem_empty + buf), 0));
-    }
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  cluster_sync_all();                                   // nobody leaves while the peer may still read its shared memory / signal its barriers
-  if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
 }
 
 // ---------------------------------------------------------------------------------------------------------------------------
@@ -749,22 +544,9 @@ __global__ void __launch_bounds__(256) segment_mean_kernel(const __half* __restr
 // ---------------------------------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFnU)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                                   const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFnU get_encode_fn_u() {
-  static EncodeTiledFnU fn = nullptr;
-  if (!fn) {
-    void* ptr = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &qres) != cudaSuccess || qres != cudaDriverEntryPointSuccess) return nullptr;
-    fn = reinterpret_cast<EncodeTiledFnU>(ptr);
-  }
-  return fn;
-}
-
 // activation map: channels-last f16 [E][HT][WD][stride], channels [0, C) of the slice starting at `base`
 static int make_act_map(CUtensorMap* map, const void* base, int C, int stride, int WD, int HT, int E, int TW, int box_rows) {
-  EncodeTiledFnU enc = get_encode_fn_u();
+  EncodeTiledFn enc = tensor_map_encoder();
   if (!enc) { set_error("cuTensorMapEncodeTiled entry point not available"); return DBA_ERR_CUDA; }
   cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)WD, (cuuint64_t)HT, (cuuint64_t)E};
   cuuint64_t strides[3] = {(cuuint64_t)stride * 2, (cuuint64_t)WD * stride * 2, (cuuint64_t)HT * WD * stride * 2};
@@ -777,7 +559,7 @@ static int make_act_map(CUtensorMap* map, const void* base, int C, int stride, i
 }
 // weight map: [taps][Ntot][Kpad] f16
 static int make_weight_map(CUtensorMap* map, const void* base, int Kpad, int Ntot, int taps, int boxn) {
-  EncodeTiledFnU enc = get_encode_fn_u();
+  EncodeTiledFn enc = tensor_map_encoder();
   if (!enc) { set_error("cuTensorMapEncodeTiled entry point not available"); return DBA_ERR_CUDA; }
   cuuint64_t dims[3] = {(cuuint64_t)Kpad, (cuuint64_t)Ntot, (cuuint64_t)taps};
   cuuint64_t strides[2] = {(cuuint64_t)Kpad * 2, (cuuint64_t)Ntot * Kpad * 2};
@@ -791,17 +573,12 @@ static int make_weight_map(CUtensorMap* map, const void* base, int Kpad, int Nto
 
 struct ConvSrc { const void* base; int C; int stride; };
 
-static int g_num_sms = 0;
-
 // one convolution launch.  src0 (+ optional src1) = channels-last sources concatenated along K; wpk = packed weights
 // [KS*KS][n_ntiles*N][Kpad] with Kpad = 64 * (kblocks(src0) + kblocks(src1)).
 template <int EPI>
 static int launch_conv(ConvParams p, ConvSrc s0, ConvSrc s1, const void* wpk, cudaStream_t st, int* slots_out = nullptr) {
-  if (!g_num_sms) {
-    int dev = 0; cudaGetDevice(&dev);
-    cudaDeviceProp prop; DBA_CHECK_CUDA(cudaGetDeviceProperties(&prop, dev), "cudaGetDeviceProperties");
-    g_num_sms = prop.multiProcessorCount;
-  }
+  DeviceInfo dev;
+  int rc = device_info(&dev); if (rc) return rc;
   p.TW = (p.WD % 64 == 0) ? 64 : 32;
   p.RM = 128 / p.TW;
   // M tiles per CTA tile: every weight stage is shared by MT tiles (and every halo row by 3 taps), so larger is better for the
@@ -810,57 +587,35 @@ static int launch_conv(ConvParams p, ConvSrc s0, ConvSrc s1, const void* wpk, cu
   // N <= 128 with a long K loop (the q convolution): 4 tiles per weight stage beat the overlapped epilogue of 2 (measured:
   // profiles/r2_conv_pipeline_experiments.txt); short K loops keep the double-buffered accumulators
   if (p.N <= 128 && p.HT >= 4 * p.RM && (s0.C + 63) / 64 + (s1.base ? (s1.C + 63) / 64 : 0) >= 4 && p.KS == 3) p.MT = 4;
-  static const int ov_mt = getenv("DBA_CONV_MT") ? atoi(getenv("DBA_CONV_MT")) : 0;          // experiment switches (tools/conv_bench.py)
-  static const int ov_as = getenv("DBA_CONV_ASTAGES") ? atoi(getenv("DBA_CONV_ASTAGES")) : 0;
-  static const int ov_bs = getenv("DBA_CONV_BSTAGES") ? atoi(getenv("DBA_CONV_BSTAGES")) : 0;
-  if (ov_mt > 0 && ov_mt * p.N <= 512 && ov_mt <= 4) p.MT = ov_mt;
   p.tiles_x = (p.WD + p.TW - 1) / p.TW;
   p.tiles_y = (p.HT + p.MT * p.RM - 1) / (p.MT * p.RM);
   p.nk0 = (s0.C + 63) / 64;
   p.nk1 = s1.base ? (s1.C + 63) / 64 : 0;
-  // CTA pairs (cta_group::2) share every weight stage: each CTA holds half of the N rows (DBA_CONV_2CTA=0 selects the single-CTA kernel)
-  static const int ov_pair = getenv("DBA_CONV_2CTA") ? atoi(getenv("DBA_CONV_2CTA")) : -1;
-  const bool use_pair = (ov_pair < 0 ? kPairDefault : ov_pair != 0) && (p.N % 32 == 0) && g_num_sms >= 2;
-  p.boxn = use_pair ? (p.N <= 256 ? p.N / 2 : 64) : (p.N <= 256 ? p.N : 128);
+  p.boxn = p.N <= 256 ? p.N : 128;
   p.nbuf = (p.MT * p.N <= 256) ? 2 : 1;
   const int box_rows = p.MT * p.RM + p.KS - 1;
   p.a_bytes = box_rows * p.TW * 128;
-  p.b_bytes = (use_pair ? p.N / 2 : p.N) * 128;
+  p.b_bytes = p.N * 128;
   // shared memory: at least 2 halo stages and 3 weight stages; what is left goes to more halo stages (up to 4: with narrow N the
   // MMAs of a stage are short and the TMA latency of the next halo tile is what the pipeline has to cover), then weight stages
   const int budget = 227 * 1024 - 2048;
   p.a_stages = 2;
   while (p.a_stages < 4 && (p.a_stages + 1) * p.a_bytes + 4 * p.b_bytes <= budget) p.a_stages++;
-  if (ov_as > 0 && ov_as <= 4) p.a_stages = ov_as;
   p.b_stages = (budget - p.a_stages * p.a_bytes) / p.b_bytes;
   if (p.b_stages > 8) p.b_stages = 8;
-  if (ov_bs > 0 && ov_bs <= 8 && p.a_stages * p.a_bytes + ov_bs * p.b_bytes <= budget) p.b_stages = ov_bs;
   if (p.b_stages < 2) { set_error("update operator: tile does not fit shared memory"); return DBA_ERR_INVALID; }
   p.slots = p.tiles_x * p.tiles_y * p.MT * 4;
   if (slots_out) *slots_out = p.slots;
   const int smem = p.a_stages * p.a_bytes + p.b_stages * p.b_bytes + 1024 + 256;
   CUtensorMap tA0, tA1, tW;
-  int rc = make_act_map(&tA0, s0.base, s0.C, s0.stride, p.WD, p.HT, p.E, p.TW, box_rows); if (rc) return rc;
+  rc = make_act_map(&tA0, s0.base, s0.C, s0.stride, p.WD, p.HT, p.E, p.TW, box_rows); if (rc) return rc;
   if (s1.base) { rc = make_act_map(&tA1, s1.base, s1.C, s1.stride, p.WD, p.HT, p.E, p.TW, box_rows); if (rc) return rc; }
   else tA1 = tA0;
   rc = make_weight_map(&tW, wpk, 64 * (p.nk0 + p.nk1), p.w_rows > 0 ? p.w_rows : p.n_ntiles * p.N, p.KS * p.KS, p.boxn); if (rc) return rc;
-  static int attr_set = 0;
-  if (attr_set < smem) {
-    DBA_CHECK_CUDA(cudaFuncSetAttribute(conv_tc_kernel<EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024), "conv_tc smem attr");
-    DBA_CHECK_CUDA(cudaFuncSetAttribute(conv_tc2_kernel<EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024), "conv_tc2 smem attr");
-    attr_set = 227 * 1024;
-  }
+  rc = kernel_setup((const void*)conv_tc_kernel<EPI>, 227 * 1024); if (rc) return rc;
   const long long total = (long long)p.n_ntiles * p.E * p.tiles_x * p.tiles_y;
   if (total <= 0) return DBA_OK;
-  if (use_pair) {
-    const long long tpn = (long long)p.E * p.tiles_x * p.tiles_y;
-    const long long pairs = (long long)p.n_ntiles * ((tpn + 1) / 2);
-    const int npairs = (int)(pairs < g_num_sms / 2 ? pairs : g_num_sms / 2);
-    conv_tc2_kernel<EPI><<<2 * npairs, kUpThreads, smem, st>>>(tA0, tA1, tW, p);
-    DBA_CHECK_LAUNCH("conv_tc2_kernel");
-    return DBA_OK;
-  }
-  const int grid = (int)(total < g_num_sms ? total : g_num_sms);
+  const int grid = (int)(total < dev.num_sms ? total : dev.num_sms);
   conv_tc_kernel<EPI><<<grid, kUpThreads, smem, st>>>(tA0, tA1, tW, p);
   DBA_CHECK_LAUNCH("conv_tc_kernel");
   return DBA_OK;

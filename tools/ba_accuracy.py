@@ -13,4 +13,4 @@ be.ba(P, D, *args, s["t0"], s["t1"], 2, s["lm"], s["ep"], False)
 P, D = P.cpu().double(), D.cpu().double()
 P64, D64 = s["poses"].double(), s["disps"].double()
 oracle.ba(P64, D64, s["intrinsics"], s["disps_sens"], s["targets"], s["weights"], s["eta"], s["ii"], s["jj"], s["t0"], s["t1"], 2, s["lm"], s["ep"], False, dtype=torch.float64)
-print("%s: pose err %.3e disp err %.3e" % (os.environ.get("DBA_SCHUR_SIMT", "0") == "1" and "simt" or "tensor-core", float((P - P64).abs().max()), float((D - D64).abs().max())))
+print("pose err %.3e disp err %.3e" % (float((P - P64).abs().max()), float((D - D64).abs().max())))

@@ -1,17 +1,12 @@
-"""Per-phase timing of the damped SPD solve (in-kernel %globaltimer stamps printed by the library when DBA_CHOL_TIMING=1) followed by a
-CUDA-event timing of 200 back-to-back solves without the stamps.  usage: python tools/chol_timing.py [n]   (DBA_CHOL_RESIDENT=0 selects
-the barrier kernel for n <= 448)."""
+"""CUDA-event timing of 200 back-to-back damped SPD solves and their error against fp64 LAPACK.
+usage: python tools/chol_timing.py [n]   (n <= 448 runs the resident-tile kernel, larger n the barrier kernel)"""
 import ctypes
 import os
-import subprocess
 import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 426
-if len(sys.argv) <= 2:       # first a child with the stamps on, then this process without them
-    env = dict(os.environ, DBA_CHOL_TIMING="1")
-    subprocess.run([sys.executable, os.path.abspath(__file__), str(n), "stamps"], env=env)
 import torch  # noqa: E402
 from droid_slam_b200 import c_api  # noqa: E402
 
@@ -31,11 +26,6 @@ def solve():
                     ctypes.c_void_p(fail.data_ptr()), ctypes.c_void_p(ws.data_ptr()), ws.numel(), None)
 
 
-if len(sys.argv) > 2:
-    for it in range(3):
-        solve()
-        torch.cuda.synchronize()
-    sys.exit(0)
 for it in range(20):
     solve()
 torch.cuda.synchronize()
@@ -50,4 +40,4 @@ Hd.diagonal().add_(0.1 + 1e-4 * Hc.diagonal())
 ref = torch.linalg.solve(Hd, bc)
 err = float((x.cpu().double() - ref).abs().max() / ref.abs().max())
 print("n=%d  %s kernel: %.1f us per solve (200 back-to-back), fail=%d, max rel err vs fp64 LAPACK %.2e"
-      % (n, "barrier" if os.environ.get("DBA_CHOL_RESIDENT") == "0" or n > 448 else "resident", 1e3 * e0.elapsed_time(e1) / 200, int(fail), err))
+      % (n, "barrier" if n > 448 else "resident", 1e3 * e0.elapsed_time(e1) / 200, int(fail), err))

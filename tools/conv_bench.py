@@ -1,5 +1,5 @@
 """Timing of the channels-last tensor-core convolution (dba_conv_nhwc) at the update operator's layer shapes, 48x64, CUDA events.
-Prints TFLOP/s per shape; the DBA_CONV_{MT,ASTAGES,BSTAGES} environment switches select pipeline variants (one process per variant)."""
+Prints TFLOP/s per shape."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -13,7 +13,6 @@ ht, wd = 48, 64
 SHAPES = {"zr": (128, 320, 3, 256), "q": (128, 320, 3, 128), "stem": (128, 0, 3, 384), "c3x3": (128, 0, 3, 128), "heads": (256, 0, 3, 32), "c1x1": (256, 0, 1, 128)}
 which = os.environ.get("CB_SHAPES", "zr,q,stem,c3x3,heads,c1x1").split(",")
 g = torch.Generator(device=DEV).manual_seed(0)
-tag = "MT=%s AS=%s BS=%s" % (os.environ.get("DBA_CONV_MT", "-"), os.environ.get("DBA_CONV_ASTAGES", "-"), os.environ.get("DBA_CONV_BSTAGES", "-"))
 for name in which:
     c0, c1, ks, n = SHAPES[name]
     x0 = torch.randn(E, ht, wd, c0, device=DEV, generator=g).half()
@@ -30,4 +29,4 @@ for name in which:
     e1.record(); torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / 5
     fl = 2.0 * E * ht * wd * n * (c0 + c1) * ks * ks
-    print("%-22s %-6s E=%d: %8.3f ms  %7.1f TFLOP/s" % (tag, name, E, ms, fl / ms / 1e9), flush=True)
+    print("%-6s E=%d: %8.3f ms  %7.1f TFLOP/s" % (name, E, ms, fl / ms / 1e9), flush=True)
